@@ -106,6 +106,25 @@ class ClockSampler(threading.Thread):
                 "power_w_max": max(float(r[2]) for r in self.rows), "samples": len(self.rows)}
 
 
+DUMP_BYTES = 64 << 20  # --dump-outputs writes at most this much in all
+
+
+def dump_outputs(out, directory):
+    """Write every tensor of the output dict `out` as <directory>/<name>.npy (float64 stays float64, everything else
+    float32).  Each array keeps at most an equal share of DUMP_BYTES: a larger one is written as the 1-D array of its
+    elements at a fixed, seeded, sorted sample of its flat indices, so two builds of the project write comparable files."""
+    import numpy as np
+    arrays = {k: v.detach() for k, v in out.items() if torch.is_tensor(v)}
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.to("cpu", torch.float64 if t.dtype == torch.float64 else torch.float32)
+        cap = DUMP_BYTES // len(arrays) // t.element_size()
+        if t.numel() > cap:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            t = t.reshape(-1)[idx]
+        np.save(os.path.join(directory, name + ".npy"), t.numpy())
+
+
 def cpu_reference_maps_per_s(workload, steps=1, warmup=0):
     """The reference's CPU path (oracle port of its forward: same torch CPU ops, all host threads) on a bounded
     sample of the workload: ONE image of the configured size per step."""
@@ -124,6 +143,7 @@ def cpu_reference_maps_per_s(workload, steps=1, warmup=0):
         out = restate.forward(sd, sample, bb, T, noise)
     dt = (time.perf_counter() - t0) / steps
     cpu_reference_maps_per_s.last_logits = out["logits"]  # image 0 of the workload: the full-resolution parity reference
+    cpu_reference_maps_per_s.last_output = out
     return 1.0 / dt, dt, f"1 image {H}x{W}, T={T}, full forward (backbone+neck+FPN+loop+decoder), fp32, {torch.get_num_threads()} threads"
 
 
@@ -141,7 +161,11 @@ def main():
                          "them every step on a side stream; blocking = ... and wait for it on the compute stream")
     ap.add_argument("--exact", action="store_true", help="exact 3-pass fp16 split everywhere (no fp8 correction products)")
     ap.add_argument("--cpu-threads", type=int, default=0, help="host threads for the CPU reference (0 = physical cores)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the output dict of the last timed step (rank 0's) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -170,10 +194,12 @@ def main():
         if rank != 0:
             return 0
         torch.set_num_threads(host_threads())
-        # bounded: one image per step, and at most ~3 minutes of timed CPU work whatever K is
-        n_timed = max(1, min(args.steps, 16))
+        # bounded: one image per step
+        n_timed = args.steps
         n_warm = min(args.warmup, 1)
         v, dt, what = cpu_reference_maps_per_s(args.workload, steps=n_timed, warmup=n_warm)
+        if args.dump_outputs:
+            dump_outputs(cpu_reference_maps_per_s.last_output, args.dump_outputs)
         what += f"; {n_timed} timed + {n_warm} warm-up executions of ONE image each (bounded sample of the {B}-image step)"
         # `steps` / `warmup` are what was EXECUTED (the request was --steps K --warmup W: see `requested`); each executed
         # step is one image, not the per-GPU batch of the config — maps/s normalises that
@@ -223,9 +249,12 @@ def main():
     # (shard.DepthGatherer), so no rank's next step queues behind a slower peer's current one
     gatherer = shard.DepthGatherer(B * world) if world > 1 and args.gather != "none" else None
 
+    last = {}
+
     def step_resident():
         with torch.no_grad():
             out = model(resident)
+        last["out"] = out
         pred = out["pred"]
         if gatherer is None:
             return pred
@@ -310,6 +339,8 @@ def main():
         sampler.start()
     ms = timed(step_resident, args.steps, "resident")
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last["out"], args.dump_outputs)  # before any later call can reuse the engine's output buffers
     if gatherer is not None:
         # the same steps WITHOUT the collective: each rank's own pace.  With it, every rank's clock stops when the slowest
         # peer has delivered its last shard, so `resident` shows one number for all ranks; this one shows the spread

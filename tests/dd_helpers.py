@@ -20,7 +20,9 @@ def load_golden(case):
 
 def build_mirror(family, steps, trained=False):
     """The product's plugin model under the golden weight seed (cached per (family, trained); steps is mutable).
-    trained=True: the trained-like regime of oracle.configs.trainedify (the `*_trained` goldens)."""
+    trained=True: the trained-like regime of oracle.configs.trainedify (the `*_trained` goldens).
+    Always returned on the CPU: GPU tests move the shared model with .to(device), the CPU tests that follow need it
+    back on the host (the head re-packs its engines' weights when their storage changes)."""
     from diffusiondepth_b200.model import get
     if (family, trained) not in _MIRRORS:
         args = configs.make_args(family, steps)
@@ -29,7 +31,7 @@ def build_mirror(family, steps, trained=False):
         _MIRRORS[(family, trained)] = configs.trainedify(m) if trained else m
     m = _MIRRORS[(family, trained)]
     m.depth_head.diffusion_inference_steps = steps
-    return m
+    return m.cpu()
 
 
 def is_trained_case(case):

@@ -3,9 +3,9 @@
 reference's `src/main.py::test()` (:404-470): get_model(args)(args) -> .cuda() -> torch.load + load_state_dict(
 ckpt['net'], strict=False) -> nn.DataParallel -> .eval() -> DataLoader(batch_size=1) -> sample.cuda() -> net(sample).
 
-CPU part: the symlinked import works; the REAL reference main.py (when /root/reference is present) runs its own test()
-on the mirror unchanged up to the first CUDA call.  GPU part: the same sequence end to end against the golden vectors
-the real reference produced."""
+CPU part: the symlinked import works; main.py's test() sequence, with the arguments the reference's own config.py
+parses, runs on the mirror up to the first CUDA call.  GPU part: the same sequence end to end against the golden
+vectors the real reference produced."""
 import copy
 import os
 import subprocess
@@ -15,7 +15,7 @@ import textwrap
 import pytest
 import torch
 
-from oracle import configs, ref_import, restate
+from oracle import configs, restate
 import dd_helpers as helpers
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -56,25 +56,29 @@ def test_mirror_imports_as_toplevel_model(tmp_path):
     assert r.returncode == 0 and "OK Diffusion_DCbase_Model" in r.stdout, r.stderr[-2000:]
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference sources not present")
-def test_reference_main_test_runs_unchanged_up_to_the_first_cuda_call(tmp_path):
-    """The reference's own src/main.py, unmodified, with `model` = the mirror: config parses the usual flags, test()
-    builds the plugin with get_model(args)(args), loads a checkpoint with load_state_dict(strict=False), wraps it in
-    nn.DataParallel, iterates a DataLoader(batch_size=1) and calls net(sample).  Without a GPU here, `.cuda()` is a no-op
-    and the forward must then fail LOUDLY in the plugin (EngineError: no CPU path) — i.e. main.py got all the way there."""
+def test_main_py_test_runs_up_to_the_first_cuda_call(tmp_path):
+    """The reference's src/main.py::test() (:404-470) on the mirror, with the Namespace the reference's config.py +
+    check_args produce for the usual flags (tests/golden/ref_main_args.json, oracle.make_golden.fixture_main_args):
+    `model` imported through the symlink, get_model(args)(args), a checkpoint through load_state_dict(strict=False),
+    nn.DataParallel, a DataLoader(batch_size=1) of the reference's sample dicts, net(sample).  With no GPU visible,
+    `.cuda()` is a no-op and the forward must then fail LOUDLY in the plugin (EngineError: no CPU path) — i.e. the
+    sequence got all the way there."""
     ckpt = tmp_path / "model_00001.pt"
     m = helpers.build_mirror("res18", 5)
     torch.save({"net": m.state_dict(), "args": None}, ckpt)
-    stub = os.path.join(ROOT, "oracle", "refstub")
     r = _run("""
-        import sys, torch
-        torch.nn.Module.cuda = lambda self, *a, **k: self          # no GPU in this container
+        import json, os, sys, torch
+        from argparse import Namespace
+        from torch import nn
+        from torch.utils.data import DataLoader, Dataset
+        torch.nn.Module.cuda = lambda self, *a, **k: self          # no GPU visible
         torch.Tensor.cuda = lambda self, *a, **k: self
-        import main                                                  # the reference's src/main.py, unmodified
         import model
-        import os
         assert model.__file__.startswith(os.environ["DD_TMP_SRC"]), model.__file__   # ... running on the mirror
-        from torch.utils.data import Dataset
+        from model import get as get_model
+        with open(sys.argv[1]) as f:
+            args = Namespace(**json.load(f), pretrain=sys.argv[2], save_dir=os.environ["DD_TMP_EXP"])
+        args.num_threads = 0
         class TwoSamples(Dataset):                                   # emits the reference's sample dict (kittidc.py:273)
             def __init__(self, args, mode): pass
             def __len__(self): return 2
@@ -83,18 +87,25 @@ def test_reference_main_test_runs_unchanged_up_to_the_first_cuda_call(tmp_path):
                 dep = torch.rand(1, 36, 52, generator=g) * 80
                 return dict(rgb=torch.randn(3, 36, 52, generator=g), dep=dep, gt=dep, K=torch.zeros(4),
                             depth_mask=dep > 0, depth_map=dep)
-        main.get_data = lambda args: TwoSamples
-        args = main.check_args(main.args_config)
-        args.num_threads = 0
-        args.save_dir = os.environ["DD_TMP_EXP"]                     # config.py derives ../experiments/<timestamp>
         try:
-            main.test(args)
+            loader_test = DataLoader(dataset=TwoSamples(args, 'test'), batch_size=1, shuffle=False,
+                                     num_workers=args.num_threads)
+            net = get_model(args)(args)
+            net.cuda()
+            checkpoint = torch.load(args.pretrain)
+            key_m, key_u = net.load_state_dict(checkpoint['net'], strict=False)
+            if key_m:
+                raise KeyError(key_m)
+            net = nn.DataParallel(net)
+            net.eval()
+            for batch, sample in enumerate(loader_test):
+                sample = {key: val.cuda() for key, val in sample.items() if val is not None}
+                with torch.no_grad():
+                    output = net(sample)
         except Exception as e:
             print("RAISED", type(e).__name__, str(e)[:120])
-        """, [_src_tree(tmp_path), stub, ref_import.REF_SRC, ROOT],
-             ["--test_only", "--model_name", "Diffusion_DCbase_", "--backbone_module", "mmbev_resnet", "--backbone_name",
-              "mmbev_res18", "--head_specify", "DDIMDepthEstimate_Res", "--inference_steps", "5", "--gpus", "0",
-              "--pretrain", str(ckpt)], DD_TMP_SRC=str(tmp_path), DD_TMP_EXP=str(tmp_path / "exp"))
+        """, [_src_tree(tmp_path), ROOT], [os.path.join(helpers.GOLDEN_DIR, "ref_main_args.json"), str(ckpt)],
+             DD_TMP_SRC=str(tmp_path), DD_TMP_EXP=str(tmp_path / "exp"), CUDA_VISIBLE_DEVICES="")
     assert "RAISED EngineError" in r.stdout and "no CPU path" in r.stdout, (r.stdout[-1500:], r.stderr[-1500:])
 
 

@@ -1,26 +1,18 @@
 """On-disk contract around the path: official-Swin key/row conversion, checkpoint ingestion, KITTI PNG values."""
+import os
+
 import numpy as np
 import pytest
 import torch
 
 from diffusiondepth_b200 import io as ddio
 from diffusiondepth_b200.model.backbone.convert_ckpt import swin_convert
-from oracle import ref_import
-
-
-def _official_like(C=8):
-    g = torch.Generator().manual_seed(0)
-    r = lambda *s: torch.randn(*s, generator=g)  # noqa: E731
-    return {"patch_embed.proj.weight": r(C, 3, 4, 4), "patch_embed.norm.weight": r(C),
-            "layers.0.blocks.0.attn.qkv.weight": r(3 * C, C), "layers.0.blocks.0.attn.relative_position_bias_table": r(169, 2),
-            "layers.0.blocks.0.mlp.fc1.weight": r(4 * C, C), "layers.0.blocks.0.mlp.fc2.bias": r(C),
-            "layers.0.blocks.0.norm1.weight": r(C), "layers.0.downsample.reduction.weight": r(2 * C, 4 * C),
-            "layers.0.downsample.norm.weight": r(4 * C), "layers.0.downsample.norm.bias": r(4 * C),
-            "norm.weight": r(8 * C), "head.weight": r(10, 8 * C)}
+from oracle import make_golden
+import dd_helpers as helpers
 
 
 def test_swin_convert_names_and_merge_order():
-    src = _official_like()
+    src = make_golden.official_swin_like()
     out = swin_convert(src)
     assert "head.weight" not in out
     for k in ("patch_embed.projection.weight", "stages.0.blocks.0.attn.w_msa.qkv.weight",
@@ -40,14 +32,13 @@ def test_swin_convert_names_and_merge_order():
     assert torch.allclose((official * g).sum(-1), (unfold * out["stages.0.downsample.norm.weight"]).sum(-1), atol=1e-5)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference sources not present")
 def test_swin_convert_matches_reference():
-    ref = ref_import.reference_modules().swin.swin_convert
-    src = _official_like()
-    a, b = ref(dict(src)), swin_convert(dict(src))
-    assert list(a) == list(b)
-    for k in a:
-        assert torch.equal(a[k], b[k]), k
+    """Against the reference's swin_convert of the same checkpoint (tests/golden/ref_swin_convert.npz)."""
+    ref = np.load(os.path.join(helpers.GOLDEN_DIR, "ref_swin_convert.npz"), allow_pickle=False)
+    b = swin_convert(make_golden.official_swin_like())
+    assert list(b) == ref["keys"].tolist()
+    for i, k in enumerate(b):
+        assert torch.equal(b[k], torch.from_numpy(ref[f"v{i}"])), k
 
 
 def test_checkpoint_ingestion_and_png(tmp_path):

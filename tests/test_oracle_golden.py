@@ -1,10 +1,12 @@
 """Pin the CPU restatement (oracle/restate.py) and the mirror's step-invariant producers against golden
-vectors generated from the REAL reference (oracle/make_golden.py); when /root/reference is present, also
-against the reference itself, live."""
+vectors generated from the REAL reference (oracle/make_golden.py)."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
-from oracle import configs, ref_import, restate
+from oracle import configs, make_golden, restate
 import dd_helpers as helpers
 
 TOL_Z = 5e-5  # fp32-vs-fp32 re-association noise on the logits (SURVEY.md §7.2: 3e-5 vs fp64 over 20 steps)
@@ -78,64 +80,51 @@ def test_denoiser_is_nonnegative_and_batch_independent():
     assert torch.allclose(e2[:1], e0, atol=1e-6)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference sources not present")
-def test_oracle_against_live_reference_swin_head():
-    """Swin *head* path (HAHI neck + FPN + upsample_fuse loop + decoder) live against the reference, fed with
-    synthetic Swin-shaped feature maps so the (slow) Swin-L backbone is not needed on CPU."""
-    from oracle import reference_runner  # noqa: F401
-    mods = ref_import.reference_modules()
-    torch.manual_seed(11)
-    head = mods.head_swin.DDIMDepthEstimate_Swin_ADDHAHI(
-        in_channels=[64, 128, 256, 512], inference_steps=3, num_train_timesteps=1000, depth_feature_dim=16,
-        loss_cfgs=[], init_cfg=None).eval()
-    with torch.no_grad():
-        head.hahineck.level_embed.zero_()
+def test_oracle_against_reference_swin_head():
+    """Swin *head* path (HAHI neck + FPN + upsample_fuse loop + decoder) against the reference's head, fed with
+    synthetic Swin-shaped feature maps so the (slow) Swin-L backbone is not needed on CPU (tests/golden/ref_swin_head.npz:
+    the reference's decoder logits and depth under the mirror head's seeded weights, oracle.make_golden.fixture_swin_head)."""
+    ref = np.load(os.path.join(helpers.GOLDEN_DIR, "ref_swin_head.npz"), allow_pickle=False)
+    head = make_golden.swin_head_mirror()
     sd = {"depth_head." + k: v for k, v in head.state_dict().items()}
-    gen = torch.Generator().manual_seed(2)
-    H, W = 40, 56
-    fp = [torch.randn(1, c, -(-H // s), -(-W // s), generator=gen) for c, s in ((192, 4), (384, 8), (768, 16), (1536, 32))]
-    gt = torch.rand(1, 1, H, W, generator=gen) * 80
-    noise = torch.randn(1, 16, H // 2, W // 2, generator=gen)
-    from oracle.reference_runner import _inject_first_randn
-    cap = {}
-    hk = head.depth_transform.conv_inv_transform[3].register_forward_hook(lambda m, a, o: cap.__setitem__("z", o))
-    with torch.no_grad(), _inject_first_randn(noise):
-        out = head(fp, gt, gt > 0, gt_depth_map=gt)
-    hk.remove()
+    ck = float(sum(v.double().abs().sum() for v in sd.values() if v.is_floating_point()))
+    assert abs(ck - float(ref["weight_checksum"])) <= 1e-9 * ck, "weights were not regenerated identically"
+    fp, gt, noise = make_golden.swin_head_inputs()
     with torch.no_grad():
         cond = restate.fpn_condition(sd, restate.hahi_neck(sd, fp))
         lat = restate.ddim_loop(sd, cond, noise, 3, "swin")
         z = restate.decode_logits(sd, lat)
-    assert (z - cap["z"]).abs().max().item() < TOL_Z
-    assert torch.allclose(restate.decode(sd, lat), out["pred"], rtol=1e-4, atol=1e-6)
+    assert (z - torch.from_numpy(ref["logits"])).abs().max().item() < TOL_Z
+    assert torch.allclose(restate.decode(sd, lat), torch.from_numpy(ref["pred"]), rtol=1e-4, atol=1e-6)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference sources not present")
-@pytest.mark.parametrize("hw,shift", [((24, 40), 0), ((24, 40), 3), ((13, 9), 3)])
-def test_window_msa_live_reference_trained_regime(hw, shift):
+@pytest.mark.parametrize("case", range(len(make_golden.WINDOW_MSA_CASES)),
+                         ids=[f"{h}x{w}-shift{s}" for (h, w), s in make_golden.WINDOW_MSA_CASES])
+def test_window_msa_against_reference_trained_regime(case):
     """The reference's own ShiftWindowMSA / WindowMSA modules (backbone/swin.py:150-189, 250-325) with NON-ZERO
-    relative-position tables, padded (24x40 -> 28x42, 13x9 -> 14x14) and shifted windows, live against (a) the
-    restatement and (b) the mirror's module — the bias / mask / roll path that the `nopretrain` factory leaves at zero."""
-    mods = ref_import.reference_modules()
-    torch.manual_seed(5)
+    relative-position tables, padded (24x40 -> 28x42, 13x9 -> 14x14) and shifted windows, against (a) the
+    restatement and (b) the mirror's module — the bias / mask / roll path that the `nopretrain` factory leaves at zero.
+    tests/golden/ref_window_msa.npz holds a seeded sample of the reference's output tokens per case; the mirror's module
+    under the same seed has the reference module's weights (checked by checksum)."""
+    ref = np.load(os.path.join(helpers.GOLDEN_DIR, "ref_window_msa.npz"), allow_pickle=False)
+    hw, shift = make_golden.WINDOW_MSA_CASES[case]
     C, heads = 96, 3
-    ref = mods.swin.ShiftWindowMSA(embed_dims=C, num_heads=heads, window_size=7, shift_size=shift).eval()
     from diffusiondepth_b200.model.backbone import swin as mirror_swin
-    mine = mirror_swin.ShiftWindowMSA(C, heads, 7, shift).eval() if hasattr(mirror_swin, "ShiftWindowMSA") else None
-    gen = torch.Generator().manual_seed(6)
+    torch.manual_seed(5)
+    mine = mirror_swin.ShiftWindowMSA(C, heads, 7, shift).eval()
+    table, x = make_golden.window_msa_inputs(hw, heads, C)
     with torch.no_grad():
-        ref.w_msa.relative_position_bias_table.copy_(torch.randn(169, heads, generator=gen) * 0.7)
-    x = torch.randn(2, hw[0] * hw[1], C, generator=gen)
+        mine.w_msa.relative_position_bias_table.copy_(table)
+    sd = mine.state_dict()
+    ck = float(sum(v.double().abs().sum() for v in sd.values() if v.is_floating_point()))
+    assert abs(ck - float(ref[f"c{case}_weight_checksum"])) <= 1e-9 * ck, "weights were not regenerated identically"
+    rows = torch.from_numpy(ref[f"c{case}_rows"])
+    want = torch.from_numpy(ref[f"c{case}_out"])
+    tol = 2e-6 * float(ref[f"c{case}_out_absmax"]) + 1e-6
+    got = restate._shift_window_msa({"a." + k: v for k, v in sd.items()}, x, hw, "a.", heads, 7, shift)
+    assert (got[:, rows] - want).abs().max().item() < tol
     with torch.no_grad():
-        want = ref(x, hw)
-    sd = {"a." + k: v for k, v in ref.state_dict().items()}
-    got = restate._shift_window_msa(sd, x, hw, "a.", heads, 7, shift)
-    assert (got - want).abs().max().item() < 2e-6 * want.abs().max().item() + 1e-6
-    if mine is not None:
-        mine.load_state_dict(ref.state_dict(), strict=True)
-        with torch.no_grad():
-            assert (mine(x, hw) - want).abs().max().item() < 2e-6 * want.abs().max().item() + 1e-6
-    # the bias really matters in this regime
-    with torch.no_grad():
-        ref.w_msa.relative_position_bias_table.zero_()
-        assert (ref(x, hw) - want).abs().max().item() > 1e-3
+        assert (mine(x, hw)[:, rows] - want).abs().max().item() < tol
+        # the bias really matters in this regime
+        mine.w_msa.relative_position_bias_table.zero_()
+        assert (mine(x, hw)[:, rows] - want).abs().max().item() > 1e-3

@@ -1,14 +1,16 @@
 """Drop-in boundary (SURVEY.md §8b): same registries / class names / ctor arguments / state_dict keys /
 output-dict keys as the reference's src/model, and no silent CPU path."""
+import os
 from argparse import Namespace
 
+import numpy as np
 import pytest
 import torch
 
 import diffusiondepth_b200 as dd
 from diffusiondepth_b200 import model as plugin
 from diffusiondepth_b200.model.registry import DEPTH_TRANSFORM, HEADS
-from oracle import configs, ref_import
+from oracle import configs
 import dd_helpers as helpers
 
 OUTPUT_KEYS = ['aff', 'blur_depth_t', 'confidence', 'ddim_loss', 'gamma', 'gt_map_t', 'guidance', 'offset', 'pred',
@@ -64,23 +66,26 @@ def test_heads_have_no_cpu_fallback():
         m.depth_head.model(torch.zeros(1, 16, 18, 26), torch.tensor(5), torch.zeros(1, 256, 18, 26), None, None, None)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference sources not present")
 @pytest.mark.parametrize("family", ["res18", "swinl", "swinl_add", "mpvit_s"])
 def test_state_dict_matches_reference_key_for_key(family):
-    f = configs.FAMILIES[family]
-    ref = ref_import.build_reference_model(ref_import.make_args(f["backbone_module"], f["backbone_name"],
-                                                                 f["head_specify"], 5))
+    """Against the reference model's state_dict layout (tests/golden/ref_state_dict_layout.npz: key, shape and dtype of
+    every entry), and a state_dict of exactly that layout loads into the mirror strictly."""
+    ref = np.load(os.path.join(helpers.GOLDEN_DIR, "ref_state_dict_layout.npz"), allow_pickle=False)
+    dtypes = {str(d): d for d in (torch.float32, torch.int64)}
+    a = {k: torch.zeros([int(s) for s in shape.split("x") if s], dtype=dtypes[dt])
+         for k, shape, dt in zip(ref[family + "_keys"].tolist(), ref[family + "_shapes"].tolist(),
+                                 ref[family + "_dtypes"].tolist())}
     mine = helpers.build_mirror(family, 5)
-    a, b = ref.state_dict(), mine.state_dict()
+    b = mine.state_dict()
     assert sorted(a) == sorted(b)
     for k in a:
         assert a[k].shape == b[k].shape and a[k].dtype == b[k].dtype, k
-    ref.load_state_dict(b, strict=True)
+    saved = {k: v.clone() for k, v in b.items()}
     mine.load_state_dict(a, strict=True)
+    mine.load_state_dict(saved, strict=True)  # build_mirror caches the model for other tests
     if family == "swinl":
         k = "depth_backbone.stages.2.blocks.1.attn.w_msa.relative_position_index"
-        mine_fresh = helpers.build_mirror(family, 5)
-        assert torch.equal(a[k], mine_fresh.state_dict()[k])
+        assert torch.equal(torch.from_numpy(ref["swinl_relative_position_index"]), b[k])
         assert len(a) == 532
 
 

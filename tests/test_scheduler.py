@@ -1,13 +1,16 @@
 """DDIM scheduler mirror: tables, timesteps, step and the collapsed coefficients the CUDA loop uses
 (reference src/model/diffusers/schedulers/scheduling_ddim.py; probe values from SURVEY.md §3.3)."""
 import math
+import os
 
+import numpy as np
 import pytest
 import torch
 
 from diffusiondepth_b200 import ddim_coefficients
 from diffusiondepth_b200.model.diffusers.schedulers.scheduling_ddim import DDIMScheduler
-from oracle import ref_import, restate
+from oracle import make_golden, restate
+import dd_helpers as helpers
 
 
 def test_tables_and_timesteps():
@@ -65,24 +68,25 @@ def test_add_noise_and_sample_prediction():
         DDIMScheduler().step(n, 10, x0)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference sources not present")
 def test_against_reference_scheduler():
-    ref = ref_import.reference_modules().scheduling_ddim.DDIMScheduler(num_train_timesteps=1000, clip_sample=False)
+    """Bit for bit against the reference's DDIMScheduler on the seeded chain of oracle.make_golden.fixture_scheduler
+    (tests/golden/ref_scheduler.npz: every step as a sha256 of its float32 bytes, the last step in full)."""
+    ref = np.load(os.path.join(helpers.GOLDEN_DIR, "ref_scheduler.npz"), allow_pickle=False)
     mine = DDIMScheduler(num_train_timesteps=1000, clip_sample=False)
-    assert torch.equal(ref.alphas_cumprod, mine.alphas_cumprod)
+    assert torch.equal(torch.from_numpy(ref["alphas_cumprod"]), mine.alphas_cumprod)
     g = torch.Generator().manual_seed(3)
     for T in (5, 20, 50):
-        ref.set_timesteps(T)
         mine.set_timesteps(T)
-        assert torch.equal(ref.timesteps, mine.timesteps)
+        assert torch.equal(torch.from_numpy(ref[f"T{T}_timesteps"]), mine.timesteps)
         x = torch.randn(1, 16, 6, 10, generator=g)
-        for t in ref.timesteps:
+        for i, t in enumerate(mine.timesteps):
             eps = torch.rand(x.shape, generator=g)
-            a = ref.step(eps, t, x, eta=0.0, use_clipped_model_output=True)
             b = mine.step(eps, t, x, eta=0.0, use_clipped_model_output=True)
-            assert torch.equal(a["prev_sample"], b["prev_sample"])
-            assert torch.equal(a["pred_original_sample"], b["pred_original_sample"])
-            x = a["prev_sample"]
+            assert make_golden.digest(b["prev_sample"]) == ref[f"T{T}_prev_sample_sha256"][i], (T, i)
+            assert make_golden.digest(b["pred_original_sample"]) == ref[f"T{T}_pred_original_sha256"][i], (T, i)
+            x = b["prev_sample"]
+        assert torch.equal(x, torch.from_numpy(ref[f"T{T}_last_prev_sample"]))
+        assert torch.equal(b["pred_original_sample"], torch.from_numpy(ref[f"T{T}_last_pred_original"]))
     t = torch.tensor([7, 300])
     x0, n = torch.randn(2, 16, 3, 3, generator=g), torch.randn(2, 16, 3, 3, generator=g)
-    assert torch.equal(ref.add_noise(x0, n, t), mine.add_noise(x0, n, t))
+    assert torch.equal(mine.add_noise(x0, n, t), torch.from_numpy(ref["add_noise"]))
