@@ -32,7 +32,7 @@ class DDBackboneConfig(C.Structure):
 ABI_VERSION = 1
 VARIANT_RES, VARIANT_SWIN = 0, 1
 FLAG_CUDA_GRAPH, FLAG_SIMT_CONV, FLAG_CHECK_RANGE, FLAG_HALO_CONV, FLAG_SWAP_NARROW, FLAG_PAIR_WIDE = 1, 2, 4, 8, 16, 32
-FLAG_STEP_DECODE, FLAG_FP8_CORR = 64, 128
+FLAG_STEP_DECODE, FLAG_FP8_CORR, FLAG_STOCHASTIC = 64, 128, 256
 STATUS = {0: "DD_OK", 1: "DD_ERR_INVALID", 2: "DD_ERR_CUDA", 3: "DD_ERR_UNSUPPORTED", 4: "DD_ERR_RANGE"}
 
 # name -> (restype, argtypes); every symbol include/dd_engine.h declares
@@ -45,6 +45,8 @@ SIGNATURES = {
     "dd_finalize_weights": (C.c_int, [C.c_void_p, C.c_void_p]),
     "dd_set_schedule": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_double),
                                   C.POINTER(C.c_double), C.c_int32]),
+    "dd_set_schedule_eta": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_double), C.POINTER(C.c_double),
+                                      C.POINTER(C.c_double), C.c_int32]),
     "dd_workspace_bytes": (C.c_size_t, [C.c_void_p]),
     "dd_enable_producers": (C.c_int, [C.c_void_p, C.POINTER(DDProducerConfig)]),
     "dd_enable_backbone": (C.c_int, [C.c_void_p, C.POINTER(DDBackboneConfig)]),
@@ -55,6 +57,8 @@ SIGNATURES = {
                                     C.c_void_p, C.c_size_t, C.c_void_p]),
     "dd_denoise_decode_steps": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dd_denoise_decode_stochastic": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "dd_denoiser_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int64), C.c_void_p,
                                       C.c_void_p, C.c_size_t, C.c_void_p]),
     "dd_decode": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),

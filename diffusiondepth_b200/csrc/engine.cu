@@ -519,6 +519,7 @@ struct dd_engine {
   // schedule
   std::vector<int64_t> ts;
   std::vector<float> cx, ce;
+  std::vector<float> sg;  // per-step sigma of stochastic DDIM (DD_FLAG_STOCHASTIC; zeros after dd_set_schedule)
   // workspace views
   void* ws = nullptr;
   float *x32 = nullptr, *Y = nullptr, *cond = nullptr, *stats[4] = {}, *mr[4] = {}, *temb_sel = nullptr;
@@ -533,13 +534,16 @@ struct dd_engine {
   bool feats_ready = false;  // dd_run_backbone has filled the neck's input planes
   bool cond_ready = false;  // dd_build_condition has filled `cond` for the next dd_denoise_decode(cond = NULL)
   // CUDA graphs (DD_FLAG_CUDA_GRAPH), captured on first use and replayed: the T-step loop, the same loop with a decode
-  // after every step (dd_denoise_decode_steps), the native backbone, the neck + FPN
-  enum { G_LOOP = 0, G_LOOP_STEPS = 1, G_BACKBONE = 2, G_COND = 3, G_COUNT = 4 };
-  cudaGraphExec_t graphs[G_COUNT] = {nullptr, nullptr, nullptr, nullptr};
-  int64_t graph_launches[G_COUNT] = {0, 0, 0, 0};  // kernel nodes per graph (added to `launches` per replay)
+  // after every step (dd_denoise_decode_steps), the native backbone, the neck + FPN, and the stochastic loop
+  // (dd_denoise_decode_stochastic) in its four shapes: G_STOCH + (decoded maps per step ? 1 : 0) + (latents per step ? 2 : 0)
+  enum { G_LOOP = 0, G_LOOP_STEPS = 1, G_BACKBONE = 2, G_COND = 3, G_STOCH = 4, G_COUNT = 8 };
+  cudaGraphExec_t graphs[G_COUNT] = {};
+  int64_t graph_launches[G_COUNT] = {};  // kernel nodes per graph (added to `launches` per replay)
   cudaStream_t cap_stream = nullptr;  // capture happens here (the caller's stream may be the legacy default stream)
   float* rgb_stage = nullptr;         // workspace copy of the image batch the backbone graph reads
   float* inter = nullptr;             // [T][B][2h][2w] per-step decoded depth (DD_FLAG_STEP_DECODE)
+  float* step_noise = nullptr;        // [T][B][P][16] staged per-step noise z (DD_FLAG_STOCHASTIC)
+  float* lat_steps = nullptr;         // [T][B][16][P] NCHW latent after every step (DD_FLAG_STOCHASTIC)
   int64_t launches = 0;
   int* status_host = nullptr;  // pinned
 };
@@ -641,6 +645,10 @@ size_t carve(dd_engine* e, void* base) {
   v->temb_sel = c.take<float>(static_cast<size_t>(g.B) * 256);
   if (e->cfg.flags & DD_FLAG_STEP_DECODE)
     v->inter = c.take<float>(static_cast<size_t>(e->cfg.num_inference_steps) * BP * 4);
+  if (e->cfg.flags & DD_FLAG_STOCHASTIC) {
+    v->step_noise = c.take<float>(static_cast<size_t>(e->cfg.num_inference_steps) * BP * 16);
+    v->lat_steps = c.take<float>(static_cast<size_t>(e->cfg.num_inference_steps) * BP * 16);
+  }
   if (e->rn.enabled || e->bb.enabled || e->mp.enabled)
     v->rgb_stage = c.take<float>(static_cast<size_t>(g.B) * 3 *
                                  (e->rn.enabled ? e->rn.H * e->rn.W : (e->mp.enabled ? e->mp.H * e->mp.W : e->bb.H * e->bb.W)));
@@ -983,8 +991,9 @@ int run_apply(dd_engine* e, int which, const float* temb, int temb_bstride, __ha
   return DD_OK;
 }
 
-// One ScheduledCNNRefine.forward + (optionally) the DDIM update.
-int run_step(dd_engine* e, const float* temb, int temb_bstride, float cx, float ce, float* eps_out, cudaStream_t st) {
+// One ScheduledCNNRefine.forward + (optionally) the DDIM update; z != nullptr adds sigma * z (stochastic DDIM).
+int run_step(dd_engine* e, const float* temb, int temb_bstride, float cx, float ce, float* eps_out, cudaStream_t st,
+             const float* z = nullptr, float sigma = 0.f) {
   const Geom g = geom_of(e->cfg);
   int rc;
   // noise_embedding.0 : x (16) -> 64, GN stats
@@ -1036,8 +1045,13 @@ int run_step(dd_engine* e, const float* temb, int temb_bstride, float cx, float 
   f.scale = kXScale;
   f.P = g.P;
   f.status = e->status;
+  f.z = z;
+  f.sigma = sigma;
   dim3 grid((g.P * 4 + 255) / 256, g.B);
-  dd::gn_relu_ddim_kernel<<<grid, 256, 0, st>>>(f);
+  if (z)
+    dd::gn_relu_ddim_stoch_kernel<<<grid, 256, 0, st>>>(f);
+  else
+    dd::gn_relu_ddim_kernel<<<grid, 256, 0, st>>>(f);
   e->launches++;
   cudaError_t err = cudaGetLastError();
   if (err != cudaSuccess) return fail(DD_ERR_CUDA, std::string("gn_relu_ddim: ") + cudaGetErrorString(err));
@@ -1953,7 +1967,19 @@ int dd_set_schedule(dd_handle h, const int64_t* timesteps, const double* c_x, co
     h->cx[i] = static_cast<float>(c_x[i]);
     h->ce[i] = static_cast<float>(c_eps[i]);
   }
+  h->sg.assign(n, 0.f);
   drop_graphs(h);
+  return DD_OK;
+}
+
+int dd_set_schedule_eta(dd_handle h, const int64_t* timesteps, const double* c_x, const double* c_eps,
+                        const double* sigma, int32_t n) {
+  if (!h || !sigma) return fail(DD_ERR_INVALID, "null argument");
+  for (int i = 0; i < n; ++i)
+    if (!(sigma[i] >= 0.0)) return fail(DD_ERR_INVALID, "sigma must be finite and >= 0");
+  int rc;
+  if ((rc = dd_set_schedule(h, timesteps, c_x, c_eps, n))) return rc;
+  for (int i = 0; i < n; ++i) h->sg[i] = static_cast<float>(sigma[i]);
   return DD_OK;
 }
 
@@ -1971,10 +1997,17 @@ static int poll_status(dd_handle h, cudaStream_t st) {
 
 // dd_denoise_decode and dd_denoise_decode_steps: the T-step loop (+ a decode after every step when depth_steps_out
 // is given: the *Vis heads' `pred_inter`, reference ..._swin_addHAHI_vis.py:130-149,289-304), then the final decode.
-static int denoise_impl(dd_handle h, const float* cond, const float* noise, float* latent_out, float* logit_out,
-                        float* depth_out, float* depth_steps_out, void* workspace, size_t workspace_bytes,
-                        void* cuda_stream) {
+// step_noise (stochastic engines only, then required): NCHW [T][B][16][h][w]; latent_steps_out (nullable, stochastic
+// engines only): NCHW [T][B][16][h][w], the latent after every step.
+static int denoise_impl(dd_handle h, const float* cond, const float* noise, const float* step_noise, float* latent_out,
+                        float* latent_steps_out, float* logit_out, float* depth_out, float* depth_steps_out,
+                        void* workspace, size_t workspace_bytes, void* cuda_stream) {
   if (!h || !noise || (!depth_out && !depth_steps_out)) return fail(DD_ERR_INVALID, "null argument");
+  const bool stoch = (h->cfg.flags & DD_FLAG_STOCHASTIC) != 0;
+  if (stoch != (step_noise != nullptr))
+    return fail(DD_ERR_INVALID, stoch ? "engine was created with DD_FLAG_STOCHASTIC: it needs step noise "
+                                        "(dd_denoise_decode_stochastic)"
+                                      : "dd_denoise_decode_stochastic needs an engine created with DD_FLAG_STOCHASTIC");
   if (!cond && !h->cond_ready) return fail(DD_ERR_INVALID, "cond is NULL but dd_build_condition has not run");
   if (!h->weights_ready) return fail(DD_ERR_INVALID, "dd_finalize_weights has not been called");
   if (static_cast<int>(h->ts.size()) != h->cfg.num_inference_steps) return fail(DD_ERR_INVALID, "dd_set_schedule has not been called");
@@ -1997,20 +2030,38 @@ static int denoise_impl(dd_handle h, const float* cond, const float* noise, floa
   h->launches += 2;
   const int T = h->cfg.num_inference_steps;
   const size_t map_elems = static_cast<size_t>(g.B) * g.P * 4;  // one decoded batch [B][2h][2w]
+  const size_t lat_elems = static_cast<size_t>(g.B) * g.P * 16;  // one latent batch [B][P][16]
   const bool steps = depth_steps_out != nullptr;
+  const bool lsteps = latent_steps_out != nullptr;
+  if (stoch) {
+    // the graph reads the noise from the workspace only: stage the caller's NCHW [T][B][16][P] as NHWC, T*B "images"
+    if ((rc = transpose_in(step_noise, h->step_noise, T * g.B, 16, g.P, st))) return rc;
+    h->launches++;
+  }
   auto loop = [&](cudaStream_t s) -> int {
     for (int i = 0; i < T; ++i) {
-      int r = run_step(h, h->temb + h->ts[i] * 256, 0, h->cx[i], h->ce[i], nullptr, s);
+      int r = stoch ? run_step(h, h->temb + h->ts[i] * 256, 0, h->cx[i], h->ce[i], nullptr, s, h->step_noise + i * lat_elems,
+                               h->sg[i])
+                    : run_step(h, h->temb + h->ts[i] * 256, 0, h->cx[i], h->ce[i], nullptr, s);
       if (r == DD_OK && steps) r = run_decoder(h, nullptr, h->inter + i * map_elems, s);
+      if (r == DD_OK && lsteps) {
+        r = transpose_out(h->x32, h->lat_steps + i * lat_elems, g.B, 16, g.P, s);
+        h->launches++;
+      }
       if (r != DD_OK) return r;
     }
     return DD_OK;
   };
   if (h->cfg.flags & DD_FLAG_CUDA_GRAPH) {
-    if ((rc = graph_run(h, steps ? dd_engine::G_LOOP_STEPS : dd_engine::G_LOOP, st, loop))) return rc;
+    const int which = stoch ? dd_engine::G_STOCH + (steps ? 1 : 0) + (lsteps ? 2 : 0)
+                            : (steps ? dd_engine::G_LOOP_STEPS : dd_engine::G_LOOP);
+    if ((rc = graph_run(h, which, st, loop))) return rc;
   } else if ((rc = loop(st))) {
     return rc;
   }
+  if (lsteps)
+    CUDA_TRY(cudaMemcpyAsync(latent_steps_out, h->lat_steps, static_cast<size_t>(T) * lat_elems * 4,
+                             cudaMemcpyDeviceToDevice, st));
   if (steps) {
     CUDA_TRY(cudaMemcpyAsync(depth_steps_out, h->inter, static_cast<size_t>(T) * map_elems * 4, cudaMemcpyDeviceToDevice, st));
     if (depth_out)
@@ -2032,13 +2083,23 @@ static int denoise_impl(dd_handle h, const float* cond, const float* noise, floa
 int dd_denoise_decode(dd_handle h, const float* cond, const float* noise, float* latent_out, float* logit_out,
                       float* depth_out, void* workspace, size_t workspace_bytes, void* cuda_stream) {
   if (!depth_out) return fail(DD_ERR_INVALID, "null argument");
-  return denoise_impl(h, cond, noise, latent_out, logit_out, depth_out, nullptr, workspace, workspace_bytes, cuda_stream);
+  return denoise_impl(h, cond, noise, nullptr, latent_out, nullptr, logit_out, depth_out, nullptr, workspace,
+                      workspace_bytes, cuda_stream);
 }
 
 int dd_denoise_decode_steps(dd_handle h, const float* cond, const float* noise, float* latent_out, float* logit_out,
                             float* depth_steps_out, void* workspace, size_t workspace_bytes, void* cuda_stream) {
   if (!depth_steps_out) return fail(DD_ERR_INVALID, "null argument");
-  return denoise_impl(h, cond, noise, latent_out, logit_out, nullptr, depth_steps_out, workspace, workspace_bytes, cuda_stream);
+  return denoise_impl(h, cond, noise, nullptr, latent_out, nullptr, logit_out, nullptr, depth_steps_out, workspace,
+                      workspace_bytes, cuda_stream);
+}
+
+int dd_denoise_decode_stochastic(dd_handle h, const float* cond, const float* noise, const float* step_noise,
+                                 float* latent_out, float* latent_steps_out, float* logit_out, float* depth_out,
+                                 float* depth_steps_out, void* workspace, size_t workspace_bytes, void* cuda_stream) {
+  if (!step_noise || (!depth_out && !depth_steps_out)) return fail(DD_ERR_INVALID, "null argument");
+  return denoise_impl(h, cond, noise, step_noise, latent_out, latent_steps_out, logit_out, depth_out, depth_steps_out,
+                      workspace, workspace_bytes, cuda_stream);
 }
 
 int dd_denoiser_forward(dd_handle h, const float* cond, const float* noisy, const int64_t* t_host, float* eps_out,

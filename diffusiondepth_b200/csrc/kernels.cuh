@@ -514,6 +514,9 @@ __global__ void __launch_bounds__(QPB * 256 / V, 12 / QPB) gn_apply_up_split_ker
 // eps = relu(gn(y6));  x <- c_x * x + c_eps * eps   (reference scheduling_ddim.py:285-326 with eta = 0,
 // collapsed; SURVEY.md §3.3).  Also refreshes the fp16 planes of x for the next step's first conv.
 // If eps_out != nullptr, only eps is written (bare denoiser call) and x is left untouched.
+// Stochastic DDIM (eta > 0, gn_relu_ddim_stoch_kernel): x <- fmaf(sigma, z, c_x * x + c_eps * eps), z = this step's
+// noise (reference scheduling_ddim.py:313-350); c_x / c_eps then carry sigma in c_eps = sqrt(1 - a_p - sigma^2) - ...
+// With sigma = 0 the update is bit-identical to gn_relu_ddim_kernel's.
 struct FinalArgs {
   const float* y;          // [B][P][16]
   const float* mean_rstd;  // [B][4][2]
@@ -526,8 +529,11 @@ struct FinalArgs {
   float cx, ce, scale;
   int P;
   int* status;
+  const float* z;          // stochastic kernel only: this step's noise [B][P][16]
+  float sigma;             // stochastic kernel only
 };
-__global__ void __launch_bounds__(256) gn_relu_ddim_kernel(const FinalArgs a) {
+template <bool STOCH>
+__device__ __forceinline__ void gn_relu_ddim_body(const FinalArgs& a) {
   const int b = blockIdx.y;
   const size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;  // float4 index within image
   if (i >= static_cast<size_t>(a.P) * 4) return;
@@ -550,12 +556,20 @@ __global__ void __launch_bounds__(256) gn_relu_ddim_kernel(const FinalArgs a) {
   }
   const float4 xv = reinterpret_cast<const float4*>(a.x)[o4];
   float xn[4] = {xv.x, xv.y, xv.z, xv.w};
+  float zn[4] = {0.f, 0.f, 0.f, 0.f};
+  if (STOCH) {
+    const float4 zv = reinterpret_cast<const float4*>(a.z)[o4];
+    zn[0] = zv.x; zn[1] = zv.y; zn[2] = zv.z; zn[3] = zv.w;
+  }
   bool ov = false;
   __align__(8) __half h[4];
   __align__(8) __half l[4];
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
-    xn[j] = a.cx * xn[j] + a.ce * e[j];
+    if (STOCH)
+      xn[j] = fmaf(a.sigma, zn[j], a.cx * xn[j] + a.ce * e[j]);
+    else
+      xn[j] = a.cx * xn[j] + a.ce * e[j];
     split_f16(xn[j], a.scale, h[j], l[j], ov);
   }
   reinterpret_cast<float4*>(a.x)[o4] = make_float4(xn[0], xn[1], xn[2], xn[3]);
@@ -563,6 +577,8 @@ __global__ void __launch_bounds__(256) gn_relu_ddim_kernel(const FinalArgs a) {
   reinterpret_cast<uint2*>(a.x_lo)[o4] = *reinterpret_cast<const uint2*>(l);
   if (ov) atomicOr(a.status, 1);
 }
+__global__ void __launch_bounds__(256) gn_relu_ddim_kernel(const FinalArgs a) { gn_relu_ddim_body<false>(a); }
+__global__ void __launch_bounds__(256) gn_relu_ddim_stoch_kernel(const FinalArgs a) { gn_relu_ddim_body<true>(a); }
 
 // ------------------------------------------------------------------ fp32 CUDA-core 3x3 conv (validation / DD_FLAG_SIMT_CONV)
 // Same operands and epilogues as the tcgen05 kernel: input fp16 hi/lo planes (x = (hi+lo)/scale), weights fp32

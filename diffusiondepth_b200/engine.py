@@ -73,7 +73,7 @@ class DenoiseEngine:
                  num_inference_steps: int, device: torch.device, cuda_graph: bool = True,
                  simt_conv: bool = False, check_range: bool = False, halo_conv: bool = True,
                  swap_narrow: bool = True, pair_wide: bool = True, step_decode: bool = False, workspace_pool=None,
-                 fp8_corr: bool = True):
+                 fp8_corr: bool = True, stochastic: bool = False):
         self.lib = _cabi.load_library()
         device = torch.device(device)
         if device.type != "cuda":
@@ -85,8 +85,10 @@ class DenoiseEngine:
         flags = (_cabi.FLAG_CUDA_GRAPH if cuda_graph else 0) | (_cabi.FLAG_SIMT_CONV if simt_conv else 0) | \
                 (_cabi.FLAG_CHECK_RANGE if check_range else 0) | (_cabi.FLAG_HALO_CONV if halo_conv else 0) | \
                 (_cabi.FLAG_SWAP_NARROW if swap_narrow else 0) | (_cabi.FLAG_PAIR_WIDE if pair_wide else 0) | \
-                (_cabi.FLAG_STEP_DECODE if step_decode else 0) | (_cabi.FLAG_FP8_CORR if fp8_corr else 0)
+                (_cabi.FLAG_STEP_DECODE if step_decode else 0) | (_cabi.FLAG_FP8_CORR if fp8_corr else 0) | \
+                (_cabi.FLAG_STOCHASTIC if stochastic else 0)
         self.fp8_corr = bool(fp8_corr)
+        self.stochastic = bool(stochastic)
         self.step_decode = bool(step_decode)
         cfg = _cabi.DDConfig(_cabi.ABI_VERSION, {"res": _cabi.VARIANT_RES, "swin": _cabi.VARIANT_SWIN}[variant],
                              self.batch, self.latent_hw[0], self.latent_hw[1], self.cond_hw[0], self.cond_hw[1],
@@ -151,10 +153,14 @@ class DenoiseEngine:
         self.backbone = (tuple(image_hw), int(embed_dims))
         self._ws = None
 
-    def set_schedule(self, timesteps, c_x, c_eps):
+    def set_schedule(self, timesteps, c_x, c_eps, sigma=None):
+        """`sigma`: per-step noise scale of stochastic DDIM (`DDIMScheduler.stochastic_coefficients`); None = 0."""
         n = len(timesteps)
-        _cabi.check(self.lib.dd_set_schedule(self._h, (C.c_int64 * n)(*[int(t) for t in timesteps]),
-                                             (C.c_double * n)(*c_x), (C.c_double * n)(*c_eps), n))
+        args = (self._h, (C.c_int64 * n)(*[int(t) for t in timesteps]), (C.c_double * n)(*c_x), (C.c_double * n)(*c_eps))
+        if sigma is None:
+            _cabi.check(self.lib.dd_set_schedule(*args, n))
+        else:
+            _cabi.check(self.lib.dd_set_schedule_eta(*args, (C.c_double * n)(*[float(v) for v in sigma]), n))
 
     # ---------------------------------------------------------------- calls
     def _stream(self) -> int:
@@ -245,6 +251,33 @@ class DenoiseEngine:
             C.c_void_p(latent.data_ptr() if want_latent else 0), C.c_void_p(logits.data_ptr() if want_logits else 0),
             C.c_void_p(steps.data_ptr()), C.c_void_p(self._aligned(ws)), ws.numel() - 1024, C.c_void_p(self._stream())))
         return steps, latent, logits
+
+    def denoise_decode_stochastic(self, cond: Optional[torch.Tensor], noise: torch.Tensor, step_noise: torch.Tensor,
+                                  want_latent=False, want_latent_steps=False, want_logits=False, want_depth_steps=False):
+        """Stochastic DDIM (engine created with stochastic=True): as `denoise_decode`, each step adding sigma_t * z_t with
+        z_t = step_noise[t] ([T,B,16,h,w]).  Returns (depth [B,1,2h,2w], latent, latent_steps [T,B,16,h,w], logits,
+        depth_steps [T,B,1,2h,2w]); the optional ones are None unless asked for (depth_steps needs step_decode=True)."""
+        if not self.stochastic:
+            raise EngineError("engine was created without stochastic=True")
+        if want_depth_steps and not self.step_decode:
+            raise EngineError("engine was created without step_decode=True")
+        B, (h, w), T = self.batch, self.latent_hw, self.steps
+        if cond is not None:
+            self._check_in(cond, (B, 256, *self.cond_hw))
+        self._check_in(noise, (B, 16, h, w))
+        self._check_in(step_noise, (T, B, 16, h, w))
+        f32 = dict(device=self.device, dtype=torch.float32)
+        depth = torch.empty(B, 1, 2 * h, 2 * w, **f32)
+        latent = torch.empty(B, 16, h, w, **f32) if want_latent else None
+        lsteps = torch.empty(T, B, 16, h, w, **f32) if want_latent_steps else None
+        logits = torch.empty_like(depth) if want_logits else None
+        dsteps = torch.empty(T, B, 1, 2 * h, 2 * w, **f32) if want_depth_steps else None
+        ptr = lambda t: C.c_void_p(t.data_ptr() if t is not None else 0)  # noqa: E731
+        ws = self._workspace()
+        _cabi.check(self.lib.dd_denoise_decode_stochastic(
+            self._h, ptr(cond), ptr(noise), ptr(step_noise), ptr(latent), ptr(lsteps), ptr(logits), ptr(depth),
+            ptr(dsteps), C.c_void_p(self._aligned(ws)), ws.numel() - 1024, C.c_void_p(self._stream())))
+        return depth, latent, lsteps, logits, dsteps
 
     def denoiser_forward(self, cond: torch.Tensor, noisy: torch.Tensor, t) -> torch.Tensor:
         """eps = ScheduledCNNRefine(noisy, t, cond); t: int or per-image sequence."""

@@ -83,6 +83,33 @@ class DDIMScheduler:
             ce.append(math.sqrt(1.0 - a_p) - math.sqrt(a_p * (1.0 - a_t) / a_t))
         return ts, cx, ce
 
+    def stochastic_coefficients(self, num_inference_steps=None, eta=0.0):
+        """(timesteps, c_x, c_eps, sigma) of the step with `eta` >= 0 (reference scheduling_ddim.py:313-350,
+        formula (16) of the DDIM paper), fp64 from the fp32 table:
+            x_{t-1} = c_x x_t + c_eps eps + sigma z,   sigma = eta sqrt((1 - a_p) / (1 - a_t) (1 - a_t / a_p)),
+            c_x = sqrt(a_p / a_t),   c_eps = sqrt(1 - a_p - sigma^2) - sqrt(a_p (1 - a_t) / a_t).
+        eta = 0 returns exactly `fused_coefficients` and sigma = 0.  Unlike the reference, which yields NaN there, an
+        eta with 1 - a_p - sigma^2 < 0 on some step (possible only for eta > 1) raises ValueError, as does eta < 0."""
+        eta = float(eta)
+        if not eta >= 0.0:
+            raise ValueError(f"eta must be >= 0, got {eta}")
+        ts, cx, ce = self.fused_coefficients(num_inference_steps)
+        if eta == 0.0:
+            return ts, cx, ce, [0.0] * len(ts)
+        stride = self._cfg["num_train_timesteps"] // self.num_inference_steps
+        acp = self.alphas_cumprod.to("cpu", torch.float64)
+        ce, sg = [], []
+        for t in ts:
+            a_t = float(acp[t])
+            a_p = float(acp[t - stride]) if t - stride >= 0 else float(self.final_alpha_cumprod)
+            s = eta * math.sqrt((1.0 - a_p) / (1.0 - a_t) * (1.0 - a_t / a_p))
+            dir2 = 1.0 - a_p - s * s
+            if dir2 < 0.0:
+                raise ValueError(f"eta = {eta} makes 1 - alpha_prev - sigma^2 negative at timestep {t}")
+            ce.append(math.sqrt(dir2) - math.sqrt(a_p * (1.0 - a_t) / a_t))
+            sg.append(s)
+        return ts, cx, ce, sg
+
     # -- one reverse step (torch; API parity with the reference, not on the CUDA hot path) -----------------
     def step(self, model_output, timestep, sample, eta=0.0, use_clipped_model_output=False, generator=None,
              variance_noise=None, return_dict=True):

@@ -52,6 +52,6 @@ class Diffusion_DCbase_Model(nn.Module):
                                weight_map=weight_map, instance_masks=instance_masks, image=img, **extra, **kwargs)
 
     def forward(self, sample):
-        extra = {'noise': sample['noise']} if 'noise' in sample else {}
+        extra = {k: sample[k] for k in ('noise', 'step_noise') if k in sample}  # seeded / sharded runs inject the draws
         return self.extract_depth(sample['rgb'], sample['depth_map'], sample['depth_mask'], sample['gt'],
                                   return_loss=True, sparse_depth=sample['dep'], **extra)

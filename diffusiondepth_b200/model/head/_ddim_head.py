@@ -28,6 +28,7 @@ from .._blocks import ConvModule, exact_fp32
 from ..diffusers.schedulers.scheduling_ddim import DDIMScheduler
 from ..ops import depth_transform as _codec  # noqa: F401  (registers the codec classes)
 from ..registry import DEPTH_TRANSFORM
+from ._pipeline import CNNDDIMPipiline, draw_step_noise
 
 FPN_DIM = 256
 MAX_ENGINES = 4  # per head: least-recently-used engines beyond this are closed (packed weights + CUDA graphs freed)
@@ -137,6 +138,7 @@ class DDIMHeadBase(nn.Module):
         #                                        backbone with every call; this is the fallback for direct head calls)
         self.capture_cond = False        # tests: keep the NCHW condition map of the last forward
         self.noise_generator: Optional[torch.Generator] = None
+        self.ddim_eta = 0.0  # eta of the DDIM sampler forward() runs (reference pipeline `eta=`); > 0: stochastic DDIM
         self._reset_engine_state()
 
     def _reset_engine_state(self):
@@ -172,6 +174,12 @@ class DDIMHeadBase(nn.Module):
         replica = super()._replicate_for_data_parallel()
         replica.__dict__['_backbone_ref'] = None
         return replica
+
+    @property
+    def pipeline(self) -> CNNDDIMPipiline:
+        """`self.pipeline(batch_size, device, dtype, shape, input_args, generator, eta, num_inference_steps, return_dict)`
+        of the reference heads (head :49, :254-303), served by this head's engines (_pipeline.py)."""
+        return CNNDDIMPipiline(self.model, self.scheduler, with_image_list=bool(self.return_intermediates))
 
     # ------------------------------------------------------------------------------------------ engine bridge
     def _engine_tensors(self):
@@ -289,27 +297,35 @@ class DDIMHeadBase(nn.Module):
                     tensors[k] = v
         return tensors
 
-    def _engine(self, batch, latent_hw, cond_hw, device, feats=None, image_hw=None, backbone=None) -> DenoiseEngine:
+    def _engine(self, batch, latent_hw, cond_hw, device, feats=None, image_hw=None, backbone=None, steps=None,
+                eta=0.0, latent_steps=False) -> DenoiseEngine:
         """feats: backbone feature maps, or a (channels, sizes) pyramid spec -> native neck/FPN;
-        image_hw: additionally run the backbone natively (`backbone`: the module holding its parameters)."""
+        image_hw: additionally run the backbone natively (`backbone`: the module holding its parameters);
+        steps: T (default diffusion_inference_steps); eta > 0 or latent_steps (the latent after every step): a
+        stochastic engine (dd_denoise_decode_stochastic) with that eta's schedule."""
         with self._lock:
-            return self._engine_locked(batch, latent_hw, cond_hw, device, feats, image_hw, backbone)
+            return self._engine_locked(batch, latent_hw, cond_hw, device, feats, image_hw, backbone,
+                                       self.diffusion_inference_steps if steps is None else int(steps), float(eta),
+                                       bool(latent_steps))
 
-    def _engine_locked(self, batch, latent_hw, cond_hw, device, feats, image_hw, backbone) -> DenoiseEngine:
+    def _engine_locked(self, batch, latent_hw, cond_hw, device, feats, image_hw, backbone, steps=None, eta=0.0,
+                       latent_steps=False) -> DenoiseEngine:
         native = feats is not None
         if native and not isinstance(feats, tuple):
             feats = ([f.shape[1] for f in feats], [tuple(f.shape[-2:]) for f in feats])
         device = torch.device(device)
-        key = (batch, tuple(latent_hw), tuple(cond_hw), str(device), self.diffusion_inference_steps,
+        steps = self.diffusion_inference_steps if steps is None else steps
+        stochastic = eta > 0 or latent_steps
+        key = (batch, tuple(latent_hw), tuple(cond_hw), str(device), steps,
                self.use_cuda_graph, native, tuple(image_hw) if image_hw is not None else None,
-               bool(self.return_intermediates), bool(self.fp8_corrections))
+               bool(self.return_intermediates), bool(self.fp8_corrections), float(eta), bool(latent_steps))
         eng = self._engines.get(key)
         if eng is None:
             pool = self._pools.setdefault(str(device), WorkspacePool(device))
-            eng = DenoiseEngine(self.variant, batch, latent_hw, cond_hw, self.diffusion_inference_steps, device,
+            eng = DenoiseEngine(self.variant, batch, latent_hw, cond_hw, steps, device,
                                 cuda_graph=self.use_cuda_graph, check_range=False,
                                 step_decode=bool(self.return_intermediates), workspace_pool=pool,
-                                fp8_corr=bool(self.fp8_corrections))
+                                fp8_corr=bool(self.fp8_corrections), stochastic=stochastic)
             if native:
                 eng.enable_producers(feats[0], feats[1], has_neck=self.has_neck)
             if image_hw is not None:
@@ -320,8 +336,11 @@ class DDIMHeadBase(nn.Module):
                     eng.enable_backbone(image_hw)
                 else:
                     eng.enable_backbone(image_hw, depths=[len(st) for st in self._backbone(backbone).layers], kind="resnet")
-            ts, cx, ce = self.scheduler.fused_coefficients(self.diffusion_inference_steps)
-            eng.set_schedule(ts, cx, ce)
+            if stochastic:
+                eng.set_schedule(*self.scheduler.stochastic_coefficients(steps, eta))
+            else:
+                ts, cx, ce = self.scheduler.fused_coefficients(steps)
+                eng.set_schedule(ts, cx, ce)
             self._engines[key] = eng
             self._packed.pop(key, None)
             while len(self._engines) > MAX_ENGINES:  # a ragged last batch / a new image size must not pile up engines
@@ -369,6 +388,24 @@ class DDIMHeadBase(nn.Module):
         tl = t.reshape(-1).tolist() if torch.is_tensor(t) else t
         return eng.denoiser_forward(cond.contiguous().float(), noisy.contiguous().float(), tl)
 
+    def sample_latents(self, cond, x_T, step_noise, eta, steps, latent_steps=False):
+        """The DDIM loop alone on the engine (the pipeline's work): cond [B,256,hc,wc], x_T [B,16,h,w], step_noise
+        [T,B,16,h,w] (None: eta = 0) -> (final latent, latent after every step [T,B,16,h,w] or None)."""
+        B = x_T.shape[0]
+        eng = self._engine(B, x_T.shape[-2:], cond.shape[-2:], x_T.device, steps=steps, eta=eta,
+                           latent_steps=latent_steps)
+        if eng.stochastic:
+            if step_noise is None:  # eta = 0 with per-step latents: sigma = 0, the noise is never weighted in
+                step_noise = torch.zeros((steps, *x_T.shape), device=x_T.device, dtype=torch.float32)
+            _, latent, lsteps, _, _ = eng.denoise_decode_stochastic(cond, x_T, step_noise.contiguous().float(),
+                                                                    want_latent=True, want_latent_steps=latent_steps)
+        else:
+            _, latent, _ = eng.denoise_decode(cond, x_T, want_latent=True)
+            lsteps = None
+        if self.check_range:
+            eng.poll_status()
+        return latent, lsteps
+
     # ------------------------------------------------------------------------------------------ condition path
     def _condition(self, fp):
         """Top-down FPN that builds the 256-channel condition map x (head :112-122 / res.py:108-118)."""
@@ -391,11 +428,20 @@ class DDIMHeadBase(nn.Module):
             return torch.randn(shape, generator=g, dtype=dtype).to(device)
         return torch.randn(shape, generator=g, device=device, dtype=dtype)
 
+    def _draw_step_noise(self, steps, shape, device, dtype, override):
+        """The stochastic loop's per-step noise [T, *shape]: `override`, or T draws in the reference's order (after x_T)."""
+        if override is not None:
+            return override.to(device=device, dtype=torch.float32).contiguous()
+        g = self.noise_generator
+        z = draw_step_noise(steps, shape, g.device if g is not None else device, dtype, g)
+        return z.to(device=device, dtype=torch.float32).contiguous()
+
     # ------------------------------------------------------------------------------------------ forward
     def forward(self, fp, depth_map, depth_mask, gt_depth_map=None, return_loss=False, noise=None, image=None,
-                backbone=None, **kwargs):
+                backbone=None, step_noise=None, **kwargs):
         """fp: backbone feature maps — or None, meaning "run the backbone natively from `image`" (the model
-        wrapper does that when `can_run_backbone` holds, and passes `backbone` = the module holding its weights)."""
+        wrapper does that when `can_run_backbone` holds, and passes `backbone` = the module holding its weights).
+        With `self.ddim_eta` > 0 the loop is stochastic DDIM; `step_noise` [T,B,16,h,w] then replaces its T draws."""
         with_backbone = fp is None
         if with_backbone:
             B, dev, dtype = image.shape[0], image.device, torch.float32
@@ -418,23 +464,33 @@ class DDIMHeadBase(nn.Module):
         else:
             cond = None
         x_T = self._draw_noise((B, 16, *latent_hw), dev, dtype, noise)
+        eta = float(self.ddim_eta)
+        z = self._draw_step_noise(self.diffusion_inference_steps, (B, 16, *latent_hw), dev, dtype, step_noise) \
+            if eta > 0 else None
         if native:  # (backbone +) neck + FPN + loop + decoder inside the engine; the condition map never leaves NHWC
             want_cond = self.capture_cond or self.training or self.eval_ddim_loss
             if with_backbone:
                 eng = self._engine(B, latent_hw, sizes[0], dev, feats=(list(self.fpn_in_channels), sizes),
-                                   image_hw=tuple(image.shape[-2:]), backbone=backbone)
+                                   image_hw=tuple(image.shape[-2:]), backbone=backbone, eta=eta)
                 eng.run_backbone(image.contiguous().float())
                 cond = eng.build_condition(None, want_cond=want_cond)
             else:
-                eng = self._engine(B, latent_hw, tuple(fp[0].shape[-2:]), dev, feats=fp)
+                eng = self._engine(B, latent_hw, tuple(fp[0].shape[-2:]), dev, feats=fp, eta=eta)
                 cond = eng.build_condition(fp, want_cond=want_cond)
             gt_map_t = eng.encode(gt_depth_map.contiguous().float())  # returned as pred_init / gt_map_t only
             loop_cond = None
         else:
-            eng = self._engine(B, latent_hw, tuple(cond.shape[-2:]), dev)
+            eng = self._engine(B, latent_hw, tuple(cond.shape[-2:]), dev, eta=eta)
             loop_cond = cond
         inter = None
-        if self.return_intermediates:  # *Vis heads: inv_t of every intermediate latent, decoded inside the graph
+        if z is not None:  # stochastic DDIM: x <- c_x x + c_eps eps + sigma_t z_t (dd_denoise_decode_stochastic)
+            refined_depth, refined_depth_t, _, logits, steps = eng.denoise_decode_stochastic(
+                loop_cond, x_T.float().contiguous(), z, want_latent=True, want_logits=self.capture_logits,
+                want_depth_steps=self.return_intermediates)
+            if self.return_intermediates:
+                inter = list(steps.unbind(0))
+                refined_depth = inter[-1]
+        elif self.return_intermediates:  # *Vis heads: inv_t of every intermediate latent, decoded inside the graph
             steps, refined_depth_t, logits = eng.denoise_decode_steps(loop_cond, x_T, want_latent=True,
                                                                       want_logits=self.capture_logits)
             inter = list(steps.unbind(0))

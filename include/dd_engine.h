@@ -21,6 +21,9 @@
  *                                    `DDIMScheduler.step`} followed by
  *                                    `DeepDepthTransformWithUpsampling.inv_t`
  *                                    (src/model/ops/depth_transform.py:33-35)
+ *   dd_set_schedule_eta / dd_denoise_decode_stochastic
+ *                                 <- the same pipeline with `eta > 0` (head :254-303 `eta=`; scheduling_ddim.py:
+ *                                    313-350): x_{t-1} = c_x * x_t + c_eps * eps + sigma_t * z_t
  *   dd_denoiser_forward           <- one bare `ScheduledCNNRefine.forward(noisy, t, cond, ...)` call
  *                                    (the operator `ddim_loss` invokes, head :207-223)
  *   dd_decode                     <- `depth_transform.inv_t(latent)` alone (the *Vis heads call it
@@ -70,13 +73,16 @@ enum dd_flags {
   DD_FLAG_SWAP_NARROW = 1 << 4, /* Cout <= 64 convs on the swapped-operand kernel (weights as A, 256 pixels as N) */
   DD_FLAG_PAIR_WIDE = 1 << 5,   /* Cout = 256 convs on CTA pairs (cluster of 2, tcgen05 cta_group::2, M = 256) */
   DD_FLAG_STEP_DECODE = 1 << 6, /* reserve workspace for dd_denoise_decode_steps (T decoded maps; the *Vis heads) */
-  DD_FLAG_FP8_CORR = 1 << 7     /* Swin variant, with HALO_CONV | PAIR_WIDE: the Cout = 256 convs (convA, convB 256->256 and
+  DD_FLAG_FP8_CORR = 1 << 7,    /* Swin variant, with HALO_CONV | PAIR_WIDE: the Cout = 256 convs (convA, convB 256->256 and
                                    noise_embedding.3 64->256) compute the correction
                                    products of the split (x_lo * w_hi, x_hi * w_lo) as e4m3 MMAs (kind::f8f6f4, K = 32) and
                                    only hi * hi in fp16: 2 pass-equivalents instead of 3, ~1.5x on the dominant kernel.
                                    Error per product ~2^-15 instead of ~2^-22 (DESIGN.md "Numerics": max |dz| 3.4e-4 on
                                    BASELINE config 3, tolerance 1e-3); activations must stay below 112 in magnitude
                                    (DD_ERR_RANGE otherwise).  Off = the exact 3-pass fp16 split everywhere. */
+  DD_FLAG_STOCHASTIC = 1 << 8   /* stochastic DDIM (eta > 0): reserve the step-noise and per-step-latent workspace regions
+                                   (2 x T*B*16*h*w fp32) for dd_denoise_decode_stochastic; dd_denoise_decode /
+                                   dd_denoise_decode_steps then fail with DD_ERR_INVALID (they have no step noise) */
 };
 
 typedef struct dd_config {
@@ -116,6 +122,12 @@ int dd_finalize_weights(dd_handle h, void* cuda_stream);
 /* Per-step timesteps (descending, as DDIMScheduler.set_timesteps produces) and the collapsed DDIM
  * coefficients; n must equal num_inference_steps. */
 int dd_set_schedule(dd_handle h, const int64_t* timesteps, const double* c_x, const double* c_eps, int32_t n);
+
+/* Stochastic DDIM: as dd_set_schedule, plus the per-step noise scale sigma_t = eta * sqrt(variance)
+ * (reference scheduling_ddim.py:313-315, formula (16)); c_eps then is sqrt(1 - a_prev - sigma^2) - sqrt(a_prev (1 - a_t)
+ * / a_t) (:321-326).  Every sigma must be >= 0.  Used by dd_denoise_decode_stochastic (dd_set_schedule leaves sigma = 0). */
+int dd_set_schedule_eta(dd_handle h, const int64_t* timesteps, const double* c_x, const double* c_eps,
+                        const double* sigma, int32_t n);
 
 /* Optional: also run the step-invariant condition producers natively — HAHI neck (attention gates off, as
  * the shipped heads configure it: src/model/necks/hahi.py:165-276) and the FPN (head :112-122) — on the same
@@ -191,6 +203,16 @@ int dd_denoise_decode(dd_handle h, const float* cond, const float* noise, float*
  * final step.  Needs DD_FLAG_STEP_DECODE at dd_create. */
 int dd_denoise_decode_steps(dd_handle h, const float* cond, const float* noise, float* latent_out, float* logit_out,
                             float* depth_steps_out, void* workspace, size_t workspace_bytes, void* cuda_stream);
+
+/* `CNNDDIMPipiline.__call__(..., eta > 0)` (head :254-303; the step's `variance_noise`, scheduling_ddim.py:329-350):
+ * the same loop with x <- c_x x + c_eps eps + sigma_t z_t.  step_noise: NCHW [T][B][16][h][w], z of step i in slice i
+ * (the i-th `variance_noise` draw of the reference loop); it is staged into the workspace before the (captured) loop runs.
+ * latent_steps_out (nullable): NCHW [T][B][16][h][w], the latent after every step (the *Vis pipelines' `image_list`);
+ * depth_steps_out (nullable, needs DD_FLAG_STEP_DECODE) as in dd_denoise_decode_steps; at least one of depth_out /
+ * depth_steps_out.  Needs DD_FLAG_STOCHASTIC.  With every sigma = 0 the outputs equal dd_denoise_decode's bit for bit. */
+int dd_denoise_decode_stochastic(dd_handle h, const float* cond, const float* noise, const float* step_noise,
+                                 float* latent_out, float* latent_steps_out, float* logit_out, float* depth_out,
+                                 float* depth_steps_out, void* workspace, size_t workspace_bytes, void* cuda_stream);
 
 /* eps = ScheduledCNNRefine(noisy, t, cond): noisy [B,16,h,w], t[b] int64 host array (one per image),
  * eps_out [B,16,h,w]. */
